@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- the driver-facing benchmark of the RetinaNet inference hot path (see DESIGN.md).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload full|postproc]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload full|postproc] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 One JSON line on rank 0.  A "step" is one pass of the hot path over one batch of synthetic input:
@@ -13,6 +13,9 @@ region; `roofline` describes the dominant kernel (live CUDA-event timing on the 
 `cpu_baseline` is the CPU oracle timed on this box's host cores (rank 0, N=1).  With N > 1 every rank
 runs the same per-GPU batch on its own images (weak scaling, image-wise sharding) and the detections
 of all ranks are gathered with one NCCL all-gather per step inside the timed region.
+Every timed loop runs exactly --steps steps.  --dump-outputs DIR writes what the last step of the measured pass
+returned (scores, boxes, classes of every image; see dump_outputs) as DIR/<name>.npy; the inputs and weights are
+seeded, so two builds of the project can be compared output for output.
 """
 import argparse
 import ctypes
@@ -222,7 +225,7 @@ class FullWorkload:
         e["k"] += 1
         main.synchronize()                                  # the step's result is on the host
 
-    def latency(self, reps=10):
+    def latency(self, reps):
         """Single-request latency of one batch, input resident, host-blocking per call (what a caller at batch 1 sees):
         CUDA-graph replay and eager launches (the eager path re-uses cached tensor maps, csrc/conv.cu)."""
         torch = self.torch
@@ -464,6 +467,26 @@ class PostprocWorkload:
                 "sample": "%d images of the same batch, all 5 levels, oracle/odtk_oracle.c decode+nms, 1 thread" % nimg}
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """arrays: name -> float32 [B, ...] numpy array, one row per image, written as out_dir/<name>.npy.  Past DUMP_LIMIT_BYTES
+    in all, the rows of a fixed seeded sample of images are written instead and their positions in the batch go to
+    out_dir/image_index.npy (float64)."""
+    import numpy as np
+    n = next(iter(arrays.values())).shape[0]
+    per_image = sum(v.nbytes for v in arrays.values()) // max(n, 1)
+    keep = min(n, DUMP_LIMIT_BYTES // max(per_image, 1))
+    if keep < n:
+        idx = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: v[idx] for k, v in arrays.items()}
+        arrays["image_index"] = idx.astype(np.float64)
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(out_dir, k + ".npy"), v)
+
+
 # BASELINE.json `configs` (and north_star's batch 1 / 8 / 32) as presets of the flags below
 CONFIGS = {
     "b1": {"workload": "full", "batch": 1}, "b8": {"workload": "full", "batch": 8}, "b32": {"workload": "full", "batch": 32},
@@ -474,7 +497,7 @@ CONFIGS = {
 }
 
 
-def postproc_sub(device, peaks, lib, rotated=False, batch=8, steps=30):
+def postproc_sub(device, peaks, lib, steps, rotated=False, batch=8):
     """decode + NMS alone (the second half of BASELINE.json's metric, configs[1]: head outputs of 8 images, fp32 NCHW entry
     points): microseconds per image, device-timed -- throughput with 3 batches in flight (CUDA graphs on 3 streams) and
     one batch at a time (eager, per-kernel event brackets) -- plus the streaming kernel's HBM roofline."""
@@ -532,7 +555,13 @@ def main():
     ap.add_argument("--no-postproc", action="store_true", help="skip the decode+NMS sub-measurement of the default line")
     ap.add_argument("--config", default=None, choices=sorted(CONFIGS),
                     help="BASELINE.json matrix presets: " + ", ".join("%s = %s" % kv for kv in sorted(CONFIGS.items())))
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the scores / boxes / classes the last measured step returned as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes what the GPU path computed: it needs --impl ours")
     if args.config:
         for k, v in CONFIGS[args.config].items():
             setattr(args, k, v)
@@ -602,6 +631,8 @@ def main():
             time.sleep(0.3)
         # pass 1: the measured value (no per-kernel events in the stream)
         ms, t0, t1 = timed(wl.step, args.steps, profile=False)
+        last = {k: t.float().cpu().numpy() for k, t in zip(("scores", "boxes", "classes"), wl.out)} \
+            if args.dump_outputs and rank == 0 else None
         clocks = sampler.stop(t0, t1) if rank == 0 else None
         # pass 2: same steps with the dominant kernel bracketed by CUDA events (roofline numbers)
         ms_prof, _, _ = timed(getattr(wl, "step_profile", wl.step), args.steps, profile=True)
@@ -672,12 +703,14 @@ def main():
             "one host-launched ncclAllGather of the packed detections per step"
     if world == 1 and args.workload == "full":
         with torch.no_grad():
-            out["latency"] = wl.latency()
+            out["latency"] = wl.latency(args.steps)
     if world == 1 and args.workload == "full" and not args.no_postproc:
         with torch.no_grad():
-            out["postproc"] = postproc_sub(device, peaks, lib, rotated=args.rotated)
+            out["postproc"] = postproc_sub(device, peaks, lib, args.steps, rotated=args.rotated)
     if world == 1 and not args.no_cpu_baseline:
         out["cpu_baseline"] = wl.cpu_baseline()
+    if last is not None:
+        dump_outputs(args.dump_outputs, last)
     print(json.dumps(out), flush=True)
     if world > 1:
         dist.destroy_process_group()

@@ -9,12 +9,14 @@ What each fixture is (reference function -> file):
   anchors.npz      odtk.box.generate_anchors / generate_anchors_rotated for strides 8..128, plus
                    the hard-coded tables of extras/cppapi/export.cpp:69-85 parsed from the source
   nms.npz          odtk.box.nms CPU path (odtk/box.py:319-367), unmodified
+  nms_uniform.npz  the same on boxes scattered uniformly over the image (3 trials, 300 boxes, 3 classes)
   decode.npz       odtk.box.decode CPU path (odtk/box.py:266-309) with '/' -> '//' on the three
                    index divisions that crash on torch >= 1.6 (ref_import.patched_cpu_decode)
   focal.npz        odtk.loss.FocalLoss forward + autograd backward (odtk/loss.py:13-18)
   snap.npz         odtk.box.snap_to_anchors (odtk/box.py:134-186), unmodified, CPU
   model_*.npz      odtk.model.Model forward (exporting=True head outputs, and the full inference
                    branch with the patched CPU decode + unmodified CPU nms)
+  model_ResNet18FPN_seed77.npz   one more ResNet18FPN head case (4 classes, state_dict seed 77, 128 x 128)
 """
 import math
 import os
@@ -88,6 +90,23 @@ def gen_nms(odtk):
     np.savez_compressed(os.path.join(OUT, "nms.npz"), **d)
 
 
+def gen_nms_uniform(odtk):
+    rng = np.random.default_rng(7)
+    d = {}
+    for k in range(3):
+        n = 300
+        ctr = rng.uniform(0, 300, (1, n, 2))
+        wh = rng.uniform(20, 100, (1, n, 2))
+        b = np.concatenate([ctr - wh / 2, ctr + wh / 2], -1).astype(np.float32)
+        s = rng.uniform(0.01, 1, (1, n)).astype(np.float32)
+        c = rng.integers(0, 3, (1, n)).astype(np.float32)
+        os_, ob, oc = odtk.box.nms(torch.from_numpy(s), torch.from_numpy(b), torch.from_numpy(c), 0.5, 100)
+        d.update({"c%d_scores" % k: s, "c%d_boxes" % k: b, "c%d_classes" % k: c, "c%d_out_scores" % k: os_.numpy(),
+                  "c%d_out_boxes" % k: ob.numpy(), "c%d_out_classes" % k: oc.numpy()})
+    d["ncases"] = np.int32(3)
+    np.savez_compressed(os.path.join(OUT, "nms_uniform.npz"), **d)
+
+
 def gen_decode(odtk):
     dec = ref_import.patched_cpu_decode()
     rng = np.random.default_rng(4321)
@@ -157,15 +176,20 @@ def gen_snap(odtk):
 def main():
     os.makedirs(OUT, exist_ok=True)
     odtk = ref_import.import_reference()
-    which = sys.argv[1:] or ["anchors", "nms", "decode", "focal", "snap", "model"]
+    which = sys.argv[1:] or ["anchors", "nms", "nms_uniform", "decode", "focal", "snap", "model", "model_seed77"]
     if "anchors" in which: gen_anchors(odtk)
     if "nms" in which: gen_nms(odtk)
+    if "nms_uniform" in which: gen_nms_uniform(odtk)
     if "decode" in which: gen_decode(odtk)
     if "focal" in which: gen_focal(odtk)
     if "snap" in which: gen_snap(odtk)
     if "model" in which:
         from oracle import gen_golden_model
         gen_golden_model.main(odtk, OUT)
+    if "model_seed77" in which:
+        from oracle import gen_golden_model
+        x = torch.randn((1, 3, 128, 128), generator=torch.Generator().manual_seed(5))
+        gen_golden_model.save(odtk, os.path.join(OUT, "model_ResNet18FPN_seed77.npz"), "ResNet18FPN", 4, 77, x)
     for f in sorted(os.listdir(OUT)):
         print(f, os.path.getsize(os.path.join(OUT, f)))
 

@@ -31,13 +31,16 @@ def reference_heads(odtk, backbone, classes, seed, x):
     return cls, box, m
 
 
+def save(odtk, path, backbone, classes, seed, x):
+    cls, box, m = reference_heads(odtk, backbone, classes, seed, x)
+    d = {"x": x.numpy(), "classes": np.int32(classes), "seed": np.int32(seed)}
+    for i, (c, b) in enumerate(zip(cls, box)):
+        d["cls%d" % i] = c.numpy()
+        d["box%d" % i] = b.numpy()
+    np.savez_compressed(path, **d)
+
+
 def main(odtk, out_dir):
     for backbone, classes, seed, shape in CASES:
         g = torch.Generator().manual_seed(seed)
-        x = torch.randn(shape, generator=g)
-        cls, box, m = reference_heads(odtk, backbone, classes, seed, x)
-        d = {"x": x.numpy(), "classes": np.int32(classes), "seed": np.int32(seed)}
-        for i, (c, b) in enumerate(zip(cls, box)):
-            d["cls%d" % i] = c.numpy()
-            d["box%d" % i] = b.numpy()
-        np.savez_compressed(os.path.join(out_dir, "model_%s.npz" % backbone), **d)
+        save(odtk, os.path.join(out_dir, "model_%s.npz" % backbone), backbone, classes, seed, torch.randn(shape, generator=g))

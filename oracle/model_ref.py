@@ -5,7 +5,7 @@ against the reference's state_dict key layout.  It is the CPU "port" used (a) to
 convolution stack (the reference itself runs nn.Conv2d: torch is the arithmetic oracle here), and
 (b) as bench.py's cpu_baseline / --impl reference leg on the GPU box, where /root/reference does
 not exist.  Pinned against the unmodified reference Model by tests/golden/model_*.npz
-(oracle/gen_golden_model.py) and, when /root/reference is mounted, by a live comparison.
+(oracle/gen_golden_model.py).
 
 Follows: odtk/model.py:125-165 (forward), odtk/backbones/fpn.py:45-61 (FPN),
 odtk/backbones/resnet.py:24-39 (feature extractor), torchvision/models/resnet.py BasicBlock :59-105,
@@ -36,15 +36,52 @@ def _conv(sd, p, x, stride=1, padding=0, groups=1):
 # The product path stores activations and weights in fp16 and accumulates in fp32 (what "fp16" means for the reference
 # too: apex AMP O2 / a TensorRT FP16 engine, SURVEY.md App. B item 10).  With fp16=True this oracle performs the SAME
 # roundings -- BatchNorm folded into the weights in fp32, weights rounded to fp16 once, every layer's output (after bias,
-# residual / upsample add and ReLU, all in fp32) rounded to fp16, head outputs kept in fp32 -- so that what remains
-# between it and the CUDA path is fp32 summation order (plus the rare 1-ulp fp16 rounding flip it causes): the conv
-# stack can then be held to 2e-3 * max|ref| and detections to 1e-3 instead of the 3e-2 an all-fp32 oracle allows.
+# residual / upsample add and ReLU, all in fp32) rounded to fp16, head outputs kept in fp32 -- and sums each convolution
+# in the product's K order (_conv_fp32_steps), so that what remains between it and the CUDA path is the rounding inside
+# one tensor-core step (plus the rare 1-ulp fp16 rounding flip it causes): the conv stack can then be held to
+# 2e-3 * max|ref| and detections to 1e-3 instead of the 3e-2 an all-fp32 oracle allows.
 def _q(x, fp16):
     return x.half().float() if fp16 else x
 
 
+def _add_rz(acc, step):
+    """fp32 accumulator + float64 step, rounded toward zero (the tensor cores truncate when they accumulate: Fasi, Higham,
+    Mikaitis, Pranesh, "Numerical behavior of NVIDIA tensor cores", PeerJ CS 2021)."""
+    s = acc.double() + step
+    f = s.float()
+    return torch.where(f.double().abs() > s.abs(), torch.nextafter(f, torch.zeros_like(f)), f)
+
+
+def _conv_fp32_steps(x, w, b, stride, padding, groups):
+    """fp16 mode: the convolution summed in the order of the product's tensor-core kernels (csrc/conv.cu) -- 64-channel
+    chunks, then taps, then the 16-channel steps of one MMA -- each step's 16 products summed exactly (float64) and added
+    to the fp32 accumulator with truncation (_add_rz), the bias added last.  torch's own CPU convolution splits its fp32
+    sums by the host's thread count, which moves the fp16 roundings downstream by as much as the parity bars allow.
+    Grouped and depthwise convolutions (at most a few hundred products per output) are summed exactly and rounded once."""
+    xd, wd = x.double(), w.double()
+    if groups > 1:
+        acc = F.conv2d(xd, wd, None, stride=stride, padding=padding, groups=groups).float()
+    else:
+        n, c, h, wi = x.shape
+        o, _, kh, kw = w.shape
+        cols = F.unfold(xd, (kh, kw), padding=padding, stride=stride)
+        cols = cols.view(n, c, kh * kw, cols.shape[-1])
+        wd = wd.reshape(o, c, kh * kw)
+        acc = torch.zeros((n, o, cols.shape[-1]), dtype=torch.float32)
+        for c64 in range(0, c, 64):
+            for tap in range(kh * kw):
+                for c0 in range(c64, min(c64 + 64, c), 16):
+                    step = torch.einsum("ncl,oc->nol", cols[:, c0:c0 + 16, tap], wd[:, c0:c0 + 16, tap])
+                    acc = _add_rz(acc, step)
+        acc = acc.view(n, o, (h + 2 * padding - kh) // stride + 1, (wi + 2 * padding - kw) // stride + 1)
+    if b is not None:
+        acc = (acc.double() + b.double().view(1, -1, 1, 1)).float()
+    return acc
+
+
 def _cb(sd, pconv, pbn, x, stride=1, padding=0, fp16=False, groups=1):
-    """conv (+ eval BatchNorm).  fp16: folded weights rounded to fp16, fp32 accumulation, fp32 shift added after."""
+    """conv (+ eval BatchNorm).  fp16: folded weights rounded to fp16, fp32 accumulation in the product's order
+    (_conv_fp32_steps), fp32 shift added after."""
     if not fp16:
         y = _conv(sd, pconv, x, stride, padding, groups)
         return _bn(sd, pbn, y) if pbn else y
@@ -53,7 +90,7 @@ def _cb(sd, pconv, pbn, x, stride=1, padding=0, fp16=False, groups=1):
         scale = sd[pbn + ".weight"] / torch.sqrt(sd[pbn + ".running_var"] + 1e-5)
         w = w * scale.view(-1, 1, 1, 1)
         b = sd[pbn + ".bias"] - sd[pbn + ".running_mean"] * scale
-    return F.conv2d(x, w.half().float(), b, stride=stride, padding=padding, groups=groups)
+    return _conv_fp32_steps(x, w.half().float(), b, stride, padding, groups)
 
 
 # MobileNetV2 (odtk/backbones/mobilenet.py:5-25 over torchvision mobilenetv2.py: features[0] 3x3 s2 conv + BN + ReLU6,

@@ -1,8 +1,8 @@
 """Import the UNMODIFIED reference package from /root/reference inside THIS container.
 
-TEST INFRASTRUCTURE ONLY.  Used by oracle/gen_golden.py (fixture generation) and by the
-not-gpu tests that re-validate the oracle whenever /root/reference is mounted.  It cannot
-travel to the GPU box; nothing under -m gpu, smoke() or bench.py may call it.
+TEST INFRASTRUCTURE ONLY.  Used by the fixture generators (oracle/gen_golden*.py), whose
+output under tests/golden/ is what the tests compare against; no test, smoke() or bench.py
+calls it.
 
 Shims (SURVEY.md section 8c): a stub `odtk._C` (the compiled extension is absent) and
 `torchvision.models.{resnet,mobilenet}.model_urls` (removed in torchvision >= 0.13).

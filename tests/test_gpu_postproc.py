@@ -1,7 +1,7 @@
 """GPU parity tests (run with -m gpu on the B200 box): the sm_100a decode / nms kernels, called
 through the C ABI (ctypes), against the CPU oracle on the same seeded inputs, against the
-committed golden fixtures, and against the reference's own CUDA kernels (oracle/_ref) when the
-prebuilt library travelled with the snapshot.
+committed golden fixtures, and against the outputs of the reference's own CUDA kernels
+(tests/golden/refcuda.npz).
 
 Bars: kept indices / classes / scores bit-exact; box coordinates within 1e-3 absolute (the only
 non-IEEE-exact operation is expf: CUDA's and glibc's differ by <= 2 ulp)."""
@@ -236,74 +236,23 @@ def test_decode_then_nms_full_pipeline_batch2():
 
 
 # ------------------------------------------------------------------------------------------------
-_REF = os.path.join(ROOT, "oracle", "_ref", "libodtk_ref.so")
-
-
-def _ref_lib():
-    L = ctypes.CDLL(_REF)
-    L.ref_decode.restype = ctypes.c_longlong
-    L.ref_nms.restype = ctypes.c_longlong
-    return L
-
-
-def _ref_decode(L, cls, deltas, anchors, stride, thresh, top_n, rotated):
-    b, ac, h, w = cls.shape
-    nbox = 6 if rotated else 4
-    a = len(anchors) // 4
-    s = torch.zeros(b, top_n, device=DEV); bx = torch.zeros(b, top_n, nbox, device=DEV); c = torch.zeros(b, top_n, device=DEV)
-    anc = (ctypes.c_float * len(anchors))(*anchors)
-    args = [b, ctypes.c_void_p(cls.data_ptr()), ctypes.c_void_p(deltas.data_ptr()), ctypes.c_void_p(s.data_ptr()),
-            ctypes.c_void_p(bx.data_ptr()), ctypes.c_void_p(c.data_ptr()), h, w, stride, a, ac // a, anc, len(anchors),
-            ctypes.c_float(thresh), top_n, int(rotated)]
-    size = L.ref_decode(*args, None, ctypes.c_longlong(0), None)
-    ws = torch.zeros(size, dtype=torch.uint8, device=DEV)
-    torch.cuda.synchronize()
-    assert L.ref_decode(*args, ctypes.c_void_p(ws.data_ptr()), ctypes.c_longlong(size), None) == 0
-    torch.cuda.synchronize()
-    return s, bx, c
-
-
-def _ref_nms(L, s, bx, c, thr, det, rotated):
-    b, n = s.shape
-    nbox = 6 if rotated else 4
-    os_ = torch.zeros(b, det, device=DEV); ob = torch.zeros(b, det, nbox, device=DEV); oc = torch.zeros(b, det, device=DEV)
-    args = [b, ctypes.c_void_p(s.data_ptr()), ctypes.c_void_p(bx.data_ptr()), ctypes.c_void_p(c.data_ptr()),
-            ctypes.c_void_p(os_.data_ptr()), ctypes.c_void_p(ob.data_ptr()), ctypes.c_void_p(oc.data_ptr()), n, det,
-            ctypes.c_float(thr), int(rotated)]
-    size = L.ref_nms(*args, None, ctypes.c_longlong(0), None)
-    ws = torch.zeros(size, dtype=torch.uint8, device=DEV)
-    torch.cuda.synchronize()
-    assert L.ref_nms(*args, ctypes.c_void_p(ws.data_ptr()), ctypes.c_longlong(size), None) == 0
-    torch.cuda.synchronize()
-    return os_, ob, oc
-
-
-@pytest.mark.skipif(not os.path.exists(_REF), reason="oracle/_ref (reference .cu build) not present")
 @pytest.mark.parametrize("rotated", [False, True])
-def test_against_reference_cuda_kernels(rotated):
+def test_against_reference_cuda_kernels(golden_dir, rotated):
     """The reference's own csrc/cuda kernels (compiled unmodified for sm_100a, --use_fast_math as
-    shipped) on the same inputs: same kept set; coordinates within 1e-3 + fast-math slack."""
-    L = _ref_lib()
-    rng = np.random.default_rng(31)
-    A = 27 if rotated else 9
-    nbox = 6 if rotated else 4
-    stride = 16
-    anchors = (oracle.generate_anchors_rotated_axis(stride, oracle.DEFAULT_RATIOS, oracle.DEFAULT_SCALES, oracle.DEFAULT_ANGLES)
-               if rotated else oracle.generate_anchors(stride, oracle.DEFAULT_RATIOS, oracle.DEFAULT_SCALES)).reshape(-1).tolist()
-    cls, deltas = _level_case(rng, 2, 10, 25, 40, A, -3.5, nbox)
-    if rotated:
-        th = rng.uniform(-np.pi / 4, np.pi / 4, size=(2, A, 25, 40))
-        d = deltas.reshape(2, A, 6, 25, 40); d[:, :, 4] = np.sin(th); d[:, :, 5] = np.cos(th)
-    tc, td = _gpu(cls), _gpu(deltas)
-    mine = _C.decode(tc, td, anchors, stride, 0.05, 1000, rotated)
-    ref = _ref_decode(L, tc, td, anchors, stride, 0.05, 1000, rotated)
-    np.testing.assert_array_equal(mine[0].cpu().numpy(), ref[0].cpu().numpy())
-    np.testing.assert_array_equal(mine[2].cpu().numpy(), ref[2].cpu().numpy())
-    np.testing.assert_allclose(mine[1].cpu().numpy(), ref[1].cpu().numpy(), atol=2e-2, rtol=0)   # __expf
-    # nms on OUR decoded boxes through both implementations
-    gs, gb, gc = _C.nms(mine[0], mine[1], mine[2], 0.5, 100, rotated)
-    rs, rb, rc = _ref_nms(L, mine[0], mine[1], mine[2], 0.5, 100, rotated)
-    gs, gb, gc, rs, rb, rc = [t.cpu().numpy() for t in (gs, gb, gc, rs, rb, rc)]
+    shipped; their outputs are stored in tests/golden/refcuda.npz by oracle/gen_golden_refcuda.py)
+    on the same inputs: same kept set; coordinates within 1e-3 + fast-math slack."""
+    from oracle import gen_golden_refcuda as refcuda
+    g = np.load(os.path.join(golden_dir, "refcuda.npz"))
+    k = "r%d_" % rotated
+    anchors, stride, cls, deltas = refcuda.decode_case(rotated)
+    mine = _C.decode(_gpu(cls), _gpu(deltas), anchors, stride, refcuda.THRESH, refcuda.TOP_N, rotated)
+    np.testing.assert_array_equal(mine[0].cpu().numpy(), g[k + "dec_scores"])
+    np.testing.assert_array_equal(mine[2].cpu().numpy(), g[k + "dec_classes"])
+    np.testing.assert_allclose(mine[1].cpu().numpy(), g[k + "dec_boxes"], atol=2e-2, rtol=0)   # __expf
+    # nms through both implementations on the decoded boxes the reference's nms was given (the product's own decode)
+    nms_in = [_gpu(g[k + "nms_in_" + n]) for n in ("scores", "boxes", "classes")]
+    gs, gb, gc = [t.cpu().numpy() for t in _C.nms(*nms_in, refcuda.NMS_THRESH, refcuda.DETECTIONS, rotated)]
+    rs, rb, rc = g[k + "nms_scores"], g[k + "nms_boxes"], g[k + "nms_classes"]
     for img in range(2):
         nk = int((rs[img] > 0).sum())
         # fast-math division can flip a decision that sits within 1 ulp of the threshold: allow

@@ -96,27 +96,17 @@ def test_iou_matches_oracle_and_golden(golden_dir):
     assert 0.9 < out[np.arange(70), np.arange(70)].min() and out.max() <= 1.01
 
 
-_REF = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "oracle", "_ref", "libodtk_ref.so")
-
-
-@pytest.mark.skipif(not os.path.exists(_REF), reason="oracle/_ref (reference .cu build) not present")
-def test_iou_matches_reference_cuda_kernel():
-    """The reference's own iou_cuda_kernel (nms_iou.cu:324-387, compiled unmodified, --use_fast_math) on the same quads:
-    same [num_anchors, num_boxes] orientation (the swapped-argument quirk) and values within fast-math slack."""
-    import ctypes
+def test_iou_matches_reference_cuda_kernel(golden_dir):
+    """The reference's own iou_cuda_kernel (nms_iou.cu:324-387, compiled unmodified, --use_fast_math; its output is stored in
+    tests/golden/refcuda.npz by oracle/gen_golden_refcuda.py) on the same quads: same [num_anchors, num_boxes] orientation
+    (the swapped-argument quirk) and values within fast-math slack."""
+    from oracle import gen_golden_refcuda as refcuda
     from retinanet_examples_b200 import _C
-    L = ctypes.CDLL(_REF)
-    L.ref_iou.restype = ctypes.c_longlong
-    rng = np.random.default_rng(8)
-    c = rng.uniform(0, 200, (300, 1, 2))
-    quads = (c + np.array([[-20, -10], [20, -10], [20, 10], [-20, 10]]) * rng.uniform(0.5, 2, (300, 1, 1))).reshape(300, 8).astype(np.float32)
-    b, a = torch.from_numpy(quads[:5].copy()).to(DEV), torch.from_numpy(quads[5:].copy()).to(DEV)
-    mine = _C.iou(b, a)[0]
-    ref = torch.zeros_like(mine)
-    torch.cuda.synchronize()
-    assert L.ref_iou(ctypes.c_void_p(b.data_ptr()), ctypes.c_void_p(a.data_ptr()), ctypes.c_void_p(ref.data_ptr()), 5, 295, None) == 0
-    torch.cuda.synchronize()
-    np.testing.assert_allclose(mine.cpu().numpy(), ref.cpu().numpy(), rtol=2e-3, atol=2e-4)
+    ref = np.load(os.path.join(golden_dir, "refcuda.npz"))["iou"]
+    b, a = refcuda.iou_case()
+    mine = _C.iou(torch.from_numpy(b).to(DEV), torch.from_numpy(a).to(DEV))[0]
+    assert tuple(mine.shape) == ref.shape
+    np.testing.assert_allclose(mine.cpu().numpy(), ref, rtol=2e-3, atol=2e-4)
     assert float(mine.max()) > 0.1
 
 

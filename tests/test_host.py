@@ -76,17 +76,19 @@ def test_level_sizes_match_survey():
 
 def test_layer_table_tool_reproduces_committed_profile(tmp_path):
     """tools/layer_table.py joins the committed ncu launch list with the engine trace of the same step; the
-    committed summary (which bench.py reads for roofline.traffic) must be what the tool computes from them."""
+    committed summary (which bench.py reads for roofline.traffic) must be what the tool computes from them
+    with the peaks the summary records."""
     import json
     import subprocess
     import sys
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
     prof = os.path.join(root, "profiles")
     out = str(tmp_path / "table")
-    subprocess.run([sys.executable, os.path.join(root, "tools", "layer_table.py"), os.path.join(prof, "r01_step_launches.csv"),
-                    os.path.join(prof, "r01_step_trace.json"), "--out", out], check=True, capture_output=True)
-    new = json.load(open(out + ".json"))["summary"]
     old = json.load(open(os.path.join(prof, "r01_layer_table.json")))["summary"]
+    subprocess.run([sys.executable, os.path.join(root, "tools", "layer_table.py"), os.path.join(prof, "r01_step_launches.csv"),
+                    os.path.join(prof, "r01_step_trace.json"), "--out", out, "--tensor-tflops", repr(old["tensor_peak_tflops"]),
+                    "--hbm-gbs", repr(old["hbm_peak_gbs"])], check=True, capture_output=True)
+    new = json.load(open(out + ".json"))["summary"]
     for k in ("launches", "sum_us", "sum_ideal_us", "conv_dram_bytes"):
         assert new[k] == old[k], k
     assert 0.5 < new["frac"] <= 1.0
@@ -136,3 +138,21 @@ def test_state_dict_layouts_match_torchvision():
         assert set(ours) == set(want), (name, sorted(set(want) ^ set(ours))[:5])
         for k, v in want.items():
             assert tuple(ours[k].shape) == tuple(v.shape), (name, k)
+
+
+def test_bench_dump_outputs_writes_float_arrays_and_caps_their_size(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one DIR/<name>.npy per returned array; past the size cap, the rows of a fixed seeded
+    sample of images and their positions in the batch (the same sample on every run)."""
+    import bench
+    rows = {"scores": np.arange(40, dtype=np.float32).reshape(10, 4), "boxes": np.ones((10, 4, 4), np.float32)}
+    bench.dump_outputs(str(tmp_path / "all"), rows)
+    assert sorted(os.listdir(tmp_path / "all")) == ["boxes.npy", "scores.npy"]
+    np.testing.assert_array_equal(np.load(tmp_path / "all" / "scores.npy"), rows["scores"])
+    monkeypatch.setattr(bench, "DUMP_LIMIT_BYTES", 3 * (16 + 64))          # room for 3 of the 10 images
+    for d in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / d), rows)
+    idx = np.load(tmp_path / "a" / "image_index.npy")
+    assert idx.dtype == np.float64 and len(idx) == 3
+    np.testing.assert_array_equal(idx, np.load(tmp_path / "b" / "image_index.npy"))
+    np.testing.assert_array_equal(np.load(tmp_path / "a" / "scores.npy"), rows["scores"][idx.astype(int)])
+    assert np.load(tmp_path / "a" / "boxes.npy").dtype == np.float32

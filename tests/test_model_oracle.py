@@ -35,12 +35,13 @@ def test_state_dict_layout_and_flop_count():
     assert sdr["cls_head.8.weight"].shape[0] == 2160 and sdr["box_head.8.weight"].shape[0] == 162
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/odtk"), reason="reference not mounted")
-def test_model_ref_against_live_reference():
-    from oracle import ref_import, gen_golden_model
-    odtk = ref_import.import_reference()
-    x = torch.randn((1, 3, 128, 128), generator=torch.Generator().manual_seed(5))
-    cls, box, _ = gen_golden_model.reference_heads(odtk, "ResNet18FPN", 4, 77, x)
-    mc, mb = model_ref.forward_heads(make_state_dict("ResNet18FPN", 4, 9, False, 77), "ResNet18FPN", x)
-    for a, b in zip(cls + box, mc + mb):
-        np.testing.assert_allclose(b.numpy(), a.numpy(), rtol=1e-4, atol=1e-5)
+def test_model_ref_against_live_reference(golden_dir):
+    """A second ResNet18FPN case (4 classes, another seed and input size): the unmodified reference Model's head outputs,
+    stored in tests/golden/model_ResNet18FPN_seed77.npz by oracle/gen_golden.py."""
+    g = np.load(os.path.join(golden_dir, "model_ResNet18FPN_seed77.npz"))
+    x = torch.from_numpy(g["x"])
+    assert torch.equal(x, torch.randn((1, 3, 128, 128), generator=torch.Generator().manual_seed(5)))
+    mc, mb = model_ref.forward_heads(make_state_dict("ResNet18FPN", int(g["classes"]), 9, False, int(g["seed"])), "ResNet18FPN", x)
+    for i in range(5):
+        np.testing.assert_allclose(mc[i].numpy(), g["cls%d" % i], rtol=1e-4, atol=1e-5)
+        np.testing.assert_allclose(mb[i].numpy(), g["box%d" % i], rtol=1e-4, atol=1e-5)

@@ -4,7 +4,6 @@ tables of extras/cppapi/export.cpp:69-85."""
 import os
 
 import numpy as np
-import pytest
 
 from oracle import oracle
 
@@ -108,21 +107,13 @@ def test_rotated_overlap_basic_properties():
     assert oracle.rotated_overlap(c, m, False) != oracle.rotated_overlap(c, m, True)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/odtk"), reason="reference not mounted")
-def test_oracle_against_live_reference_nms():
-    """When the reference is mounted (build container) re-run its CPU nms on fresh seeds."""
-    import torch
-    from oracle import ref_import
-    odtk = ref_import.import_reference()
-    rng = np.random.default_rng(7)
-    for trial in range(3):
-        n = 300
-        ctr = rng.uniform(0, 300, (1, n, 2))
-        wh = rng.uniform(20, 100, (1, n, 2))
-        b = np.concatenate([ctr - wh / 2, ctr + wh / 2], -1).astype(np.float32)
-        s = rng.uniform(0.01, 1, (1, n)).astype(np.float32)
-        c = rng.integers(0, 3, (1, n)).astype(np.float32)
-        rs, rb, rc = [t.numpy() for t in odtk.box.nms(torch.from_numpy(s), torch.from_numpy(b), torch.from_numpy(c), 0.5, 100)]
+def test_oracle_against_live_reference_nms(golden_dir):
+    """The reference's CPU nms (odtk.box.nms, unmodified) on boxes scattered uniformly over the image, 3 seeded trials:
+    tests/golden/nms_uniform.npz (oracle/gen_golden.py)."""
+    g = np.load(os.path.join(golden_dir, "nms_uniform.npz"))
+    for k in range(int(g["ncases"])):
+        s, b, c = g["c%d_scores" % k], g["c%d_boxes" % k], g["c%d_classes" % k]
+        rs, rb = g["c%d_out_scores" % k], g["c%d_out_boxes" % k]
         os_, ob, oc = oracle.nms(s, b, c, 0.5, 100)
         nk = int((rs[0] > 0).sum())
         np.testing.assert_array_equal(os_[0][:nk], rs[0][:nk])

@@ -1,7 +1,9 @@
 """Join an ncu per-launch CSV of one step (tools/capture_step.py) with the engine trace of the same step:
 per-launch duration, DRAM bytes and tensor-pipe activity next to the launch's algorithmic FLOPs / bytes and its
 layer-wise speed of light max(FLOPs / tensor peak, bytes / HBM peak).
-    python tools/layer_table.py launches.csv step_trace.json [--out profiles/rNN_layer_table]"""
+    python tools/layer_table.py launches.csv step_trace.json [--out profiles/rNN_layer_table] [--tensor-tflops T --hbm-gbs B]
+The peaks default to MEASURED_PEAKS.json at the repository root (bf16_tflops_sustained or bf16_tflops, hbm_gbs), measured on
+the GPU the capture was taken on; a committed table records the peaks it was computed with."""
 import argparse
 import collections
 import csv
@@ -18,9 +20,14 @@ def main():
     ap.add_argument("csv")
     ap.add_argument("trace")
     ap.add_argument("--out", default=None)
+    ap.add_argument("--tensor-tflops", type=float, default=None, help="tensor-pipe peak, TFLOP/s")
+    ap.add_argument("--hbm-gbs", type=float, default=None, help="HBM peak, GB/s")
     args = ap.parse_args()
-    peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
-    tf, bw = peaks.get("bf16_tflops_sustained") or peaks["bf16_tflops"], peaks["hbm_gbs"]
+    tf, bw = args.tensor_tflops, args.hbm_gbs
+    if tf is None or bw is None:
+        peaks = json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
+        tf = tf or peaks.get("bf16_tflops_sustained") or peaks["bf16_tflops"]
+        bw = bw or peaks["hbm_gbs"]
     lines = [l for l in open(args.csv) if l.startswith('"')]
     rows = collections.OrderedDict()
     for r in csv.DictReader(lines):
